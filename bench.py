@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            (torchrun launches N>1, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W
     python bench.py --workload {marigold,normals,geowizard,train} [--res R] [--batch B]      (BASELINE.json configs 2-5)
+    python bench.py ... --dump-outputs DIR        (+ what the last timed step returned, as DIR/<name>.npy)
 
 Default workload = BASELINE.json configs[1]: marigold-e2e-ft-depth inference, bs=8 per GPU, fp16 operands,
 processing_res=768, 1 denoising step, zeros noise, synthetic 3x768x768 RGB, seeded random weights.
@@ -35,6 +36,30 @@ sys.path.insert(0, ROOT)
 # tensor-pipe FLOPs (2*MAC) per image, SURVEY.md §8(d): UNet / VAE enc / VAE dec
 TFLOP_PER_IMAGE = {768: 10.501, 512: 4.429, 384: 2.444, 256: 1.10, 128: 0.28, 64: 0.07}
 METRIC = "images_per_sec_768x768_depth"
+DUMP_BYTES = 64 * 10 ** 6          # --dump-outputs writes at most this; larger outputs are stored as a fixed seeded sample
+
+
+def dump_outputs(arrays, out_dir, seed=0):
+    """Write every array as <out_dir>/<name>.npy in float32.  If together they exceed DUMP_BYTES, each keeps the same
+    share of its elements, at flat indices drawn by a generator seeded with `seed` and stored in index order: runs with
+    the same arguments store the same positions, so two builds can be compared element for element."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.numel() for a in arrays.values())
+    cap = (DUMP_BYTES - 1024 * len(arrays)) // 4          # float32 elements, leaving room for the .npy headers
+    info = {}
+    for name, a in arrays.items():
+        a = a.detach().float().cpu()
+        n = a.numel()
+        info[name] = {"shape": list(a.shape), "stored": "all"}
+        if total > cap:
+            k = n * cap // total
+            idx = torch.randperm(n, generator=torch.Generator().manual_seed(seed))[:k].sort().values
+            a = a.reshape(-1)[idx]
+            info[name]["stored"] = f"{k} of {n} elements at seeded flat indices (torch.randperm seed {seed}), ascending"
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
+    return info
 
 
 def shard_range(total, rank, world):
@@ -419,14 +444,17 @@ def run_engine(args):
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = None                        # what the last timed step returned
+
     def timed(fn, steps, time_conv=False):
+        nonlocal last
         ops.STATS.reset()
         ops.STATS.time_kind = ("gemm" if args.dump_shapes else "conv") if time_conv else None
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            last = fn()
         e1.record()
         barrier()
         ops.STATS.time_kind = None
@@ -441,6 +469,14 @@ def run_engine(args):
     launches = ops.STATS.launches
     total_flops = sum(ops.STATS.flops.values())
     flops_by_kind = {k: v / args.steps for k, v in ops.STATS.flops.items()}
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # what single_infer handed back in the last timed step
+        if wl == "geowizard":                          # infer() concatenates its (depth, normal)
+            arrays = {"depth": last[:, :1], "normal": last[:, 1:]}
+        else:
+            arrays = {"normals" if wl == "normals" else "depth": last}
+        dumped = {"dir": os.path.abspath(args.dump_outputs), "arrays": dump_outputs(arrays, args.dump_outputs)}
 
     # ---- timed region B (roofline leg): the same step launched eagerly so every implicit-GEMM conv
     # launch can be bracketed with CUDA events on the launching stream
@@ -572,6 +608,8 @@ def run_engine(args):
             out["unet_tensor_frac"] = unet_flops / (unet_ms / 1e3) / 1e12 / peak
         if fast is not None:
             out["fast_mode"] = fast
+        if dumped is not None:
+            out["dumped_outputs"] = dumped
 
     # ---- BASELINE.json configs[2]: the training step with its gradient all-reduce.  Every rank runs it in a CHILD
     # process with its own process group (MASTER_PORT + 1): a fault or a stuck collective in the training leg can then
@@ -590,7 +628,7 @@ def run_engine(args):
         if world > 1:
             dist.barrier()
             dist.destroy_process_group()
-        t = _train_subprocess(world, rank, local)
+        t = _train_subprocess(world, rank, local, args.steps, max(args.warmup, 4))
         if rank == 0:
             if isinstance(t, dict):
                 t["gpu_free_gb_at_start"] = free_b / 2 ** 30
@@ -611,16 +649,17 @@ def run_engine(args):
         dist.destroy_process_group()
 
 
-def _train_subprocess(world, rank, local, timeout_s=420):
-    """Run `bench.py --workload train` for this rank in a child process (own NCCL group on MASTER_PORT + 1)."""
+def _train_subprocess(world, rank, local, steps, warmup, timeout_s=420):
+    """Run `bench.py --workload train --steps steps` for this rank in a child process (own NCCL group on
+    MASTER_PORT + 1)."""
     env = dict(os.environ)
     env.update(RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(local),
                MASTER_ADDR=env.get("MASTER_ADDR", "127.0.0.1"), MASTER_PORT=str(int(env.get("MASTER_PORT", "29500")) + 1))
     for k in ("TORCHELASTIC_RUN_ID", "TORCHELASTIC_RESTART_COUNT", "TORCHELASTIC_MAX_RESTARTS",
               "TORCHELASTIC_USE_AGENT_STORE", "TORCH_NCCL_ASYNC_ERROR_HANDLING"):
         env.pop(k, None)                       # the child rendezvous is a plain env:// TCP store on the new port
-    cmd = [sys.executable, os.path.abspath(__file__), "--workload", "train", "--gpus", str(world), "--steps", "5",
-           "--warmup", "4", "--res", "768", "--batch", "2"]
+    cmd = [sys.executable, os.path.abspath(__file__), "--workload", "train", "--gpus", str(world), "--steps", str(steps),
+           "--warmup", str(warmup), "--res", "768", "--batch", "2"]
     try:
         p = subprocess.Popen(cmd, env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True)
         try:
@@ -656,7 +695,12 @@ def main():
     ap.add_argument("--no-train", action="store_true", help="skip the configs[2] training-step leg of the default line")
     ap.add_argument("--no-fast", action="store_true", help="skip the fp16-stream timing of the default line")
     ap.add_argument("--dump-shapes", action="store_true", help="write per-shape conv timings to gpurun_out/")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float32, rank 0; "
+                         "a fixed seeded sample when above 64 MB in all; inputs and weights are seeded)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "train"):
+        ap.error("--dump-outputs covers the engine's inference workloads")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "train":

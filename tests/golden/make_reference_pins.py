@@ -1,6 +1,6 @@
-"""Generate tests/golden/reference_pins.pt by RUNNING THE REFERENCE'S OWN CODE (imported by path from
-/root/reference, read-only) on seeded inputs.  Only the reference files that import without diffusers can be
-run here (VERDICT r1 weak #2):
+"""Generate tests/golden/reference_pins.pt by RUNNING THE REFERENCE'S OWN CODE (imported by path from a
+checkout of diffusion-e2e-ft, read-only) on seeded inputs.  Only the reference files that import without diffusers
+can be run:
 
     training/util/loss.py                        ScaleAndShiftInvariantLoss, AngularLoss   (+ autograd gradients)
     training/util/unet_prep.py                   replace_unet_conv_in
@@ -10,10 +10,11 @@ run here (VERDICT r1 weak #2):
     Marigold/src/util/alignment.py               align_depth_least_square
 
 The UNet / VAE arithmetic itself lives in diffusers==0.30.2 (absent, not installable offline) and stays pinned only
-by the oracle restatement (SURVEY.md §8c).  /root/reference does not exist on the GPU box, so the outputs are
-committed as a small fixture and tests/test_reference_pins.py compares the oracle AND the CUDA kernels with it.
+by the oracle restatement (SURVEY.md §8c).  The tests run without the reference, so the outputs are committed as a
+small fixture and tests/test_reference_pins.py compares the oracle AND the CUDA kernels with it.
 
-    python tests/golden/make_reference_pins.py
+    python tests/golden/make_reference_pins.py <checkout>            -> reference_pins.pt
+    python tests/golden/make_reference_pins.py --record <checkout>   -> reference_recorded.npz (see record())
 """
 import importlib.util
 import os
@@ -22,7 +23,7 @@ import sys
 import numpy as np
 import torch
 
-REF = "/root/reference"
+REF = None                 # the reference checkout, from the command line
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -137,7 +138,27 @@ def main():
     print("wrote", path, os.path.getsize(path), "bytes")
 
 
+def record():
+    """Re-run two reference functions on the inputs stored in reference_pins.pt and keep their outputs in
+    reference_recorded.npz, a record separate from the fixture: tests/test_reference_pins.py checks the fixture's
+    outputs against it bit for bit, so a regenerated or edited fixture cannot drift from what the reference computes."""
+    loss = load_ref("training/util/loss.py", "ref_loss")
+    nens = load_ref("GeoWizard/geowizard/utils/normal_ensemble.py", "ref_normal_ensemble")
+    pins = torch.load(os.path.join(HERE, "reference_pins.pt"))
+    s = pins["ssi"]
+    rec = {"ssi_loss": loss.ScaleAndShiftInvariantLoss()(s["pred"], s["target"], s["mask"]).detach().numpy()}
+    for name, case in pins["ensemble_normals"].items():
+        rec[f"ensemble_normals_{name}"] = nens.ensemble_normals(case["preds"]).numpy()
+    path = os.path.join(HERE, "reference_recorded.npz")
+    np.savez(path, **rec)
+    print("wrote", path, os.path.getsize(path), "bytes")
+
+
 if __name__ == "__main__":
-    if not os.path.isdir(REF):
-        sys.exit("needs /root/reference (run in the build container, not on the GPU box)")
-    main()
+    if len(sys.argv) < 2 or not os.path.isdir(sys.argv[-1]):
+        sys.exit("usage: make_reference_pins.py [--record] <checkout of diffusion-e2e-ft>")
+    REF = sys.argv[-1]
+    if "--record" in sys.argv[1:-1]:
+        record()
+    else:
+        main()
